@@ -12,10 +12,12 @@ bytes in and planar f32 pixels copied back to pinned host memory every step.
   python bench.py --impl reference      # CPU arm: the oracle (port of jxl-oxide's generic path)
 """
 import argparse
+import ctypes
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -34,19 +36,31 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 # ----------------------------------------------------------------------------------------------
 # workloads
-def synth_frame(w, h, seed, distance=1.0, extra=()):
-    """Synthetic encoded frame from tools/synth_enc.cc (built on demand; cached under bench_data/)."""
-    tool = os.path.join(ROOT, "tools", "_build_synth_enc")
+SYNTH_TOOL = os.path.join(ROOT, "tools", "_build_synth_enc")
+_synth_dir = None
+
+
+def build_synth_tool():
+    """Compiles tools/synth_enc.cc (build() does this, so that the benchmark can run from a read-only tree)."""
     src = os.path.join(ROOT, "tools", "synth_enc.cc")
+    if os.path.exists(SYNTH_TOOL) and os.path.getmtime(SYNTH_TOOL) >= os.path.getmtime(src):
+        return
     host = os.path.join(ROOT, "jxl_oxide_b200", "csrc", "host")
-    if not os.path.exists(tool) or os.path.getmtime(tool) < os.path.getmtime(src):
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-o", tool, src] +
-                              [os.path.join(host, f) for f in ("entropy.cc", "frame_syntax.cc", "modular_syntax.cc", "headers.cc")])
-    os.makedirs(os.path.join(ROOT, "bench_data"), exist_ok=True)
+    subprocess.check_call(["g++", "-std=c++17", "-O2", "-o", SYNTH_TOOL, src] +
+                          [os.path.join(host, f) for f in ("entropy.cc", "frame_syntax.cc", "modular_syntax.cc", "headers.cc")])
+
+
+def synth_frame(w, h, seed, distance=1.0, extra=()):
+    """Synthetic encoded frame from tools/synth_enc.cc: the same bytes for the same arguments. Frames are cached for the
+    life of the process in a temporary directory, not in the tree."""
+    global _synth_dir
+    build_synth_tool()
+    if _synth_dir is None:
+        _synth_dir = tempfile.TemporaryDirectory(prefix="jxlb_synth_")
     tag = "".join(extra).replace("-", "")
-    path = os.path.join(ROOT, "bench_data", f"synth_{w}x{h}_d{distance}_s{seed}{tag}.jxl")
+    path = os.path.join(_synth_dir.name, f"synth_{w}x{h}_d{distance}_s{seed}{tag}.jxl")
     if not os.path.exists(path):
-        subprocess.check_call([tool, "--width", str(w), "--height", str(h), "--seed", str(seed), "--distance", str(distance),
+        subprocess.check_call([SYNTH_TOOL, "--width", str(w), "--height", str(h), "--seed", str(seed), "--distance", str(distance),
                                "-o", path] + list(extra), stderr=subprocess.DEVNULL)
     with open(path, "rb") as f:
         return f.read()
@@ -412,6 +426,8 @@ def run_ours(args, rank, world, local_rank):
     e2e_value = total_px / (ms_e2e / args.steps / 1e3) / 1e6
     e2e_u8_value = total_px / (ms_e2e_u8 / args.steps / 1e3) / 1e6
     u8_bytes = px_per_frame * 3
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pipe, slots, w, h, args.dump_outputs)
     pipe.close()
     if dist is not None:
         dist.barrier()
@@ -511,6 +527,36 @@ def run_ours(args, rank, world, local_rank):
     if gather is not None:
         line["gather"] = gather
     print(json.dumps(line))
+
+
+def dump_outputs(pipe, slots, w, h, out_dir):
+    """--dump-outputs: the planar f32 frame (channels, h, w) a caller of the timed path receives, for every frame of one
+    step, as out_dir/frame_<k>.npy. The timed steps leave their frames in HBM and release them, so the step is decoded
+    once more through the same pipeline with each frame copied to host memory; the inputs and the decode are
+    deterministic, so these are the last timed step's outputs. Every frame is sampled at the same seeded pixel positions,
+    keeping the files within DUMP_BYTES in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    for k, slot in enumerate(slots):
+        pipe.submit(slot=slot, mode=pipe.OUT_PLANAR_F32, tag=k)
+    pos = None
+    while pipe.in_flight:
+        k, addr, nbytes = pipe.wait(want_output=True)
+        try:
+            planes = np.ctypeslib.as_array((ctypes.c_float * (nbytes // 4)).from_address(addr)).reshape(-1, w * h)
+            if pos is None:
+                pos = dump_positions(w * h, planes.shape[0], len(slots))
+            np.save(os.path.join(out_dir, f"frame_{k:03d}.npy"), planes[:, pos])
+        finally:
+            pipe.release_output(addr)
+
+
+DUMP_BYTES = 48 << 20
+
+
+def dump_positions(npx, channels, nframes):
+    """Sorted pixel indices of the --dump-outputs sample: all of a frame when it fits, else a seeded subset."""
+    n = min(npx, DUMP_BYTES // (nframes * channels * 4))
+    return np.sort(np.random.default_rng(0).choice(npx, size=n, replace=False))
 
 
 def pipe_workers(args):
@@ -687,7 +733,13 @@ def main():
                     help="HF coefficient schedule = streams per CTA: 0 (= 4) / 8 / 16 one warp per stream, 32 / 64 / 128 one "
                          "thread per stream; auto = the fixed default (HF_STREAMS_PER_CTA). JXLB_HF_LANES in the environment "
                          "overrides.")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frames of one step as DIR/frame_<k>.npy: planar f32 "
+                         "(channels, samples), the same seeded sample of pixels in every frame, at most %d MiB in all"
+                         % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
